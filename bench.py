@@ -4,6 +4,7 @@ dominant kernel and the reference's CPU path timed beside it.
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port), rank 0
+  python bench.py ... --dump-outputs DIR                   # also write the proofs of the last timed step
 
 A "step" is one full proof (Prover.prove rounds 1-5, 9 KZG commitments) of a synthetic 2^20-gate circuit
 (plonkathon_b200/synthetic.py, seeded) under a structured test SRS generated on the device.
@@ -31,6 +32,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 TAU = 0x1234567890ABCDEF1234567890ABCDEF1234567890ABCDEF  # fixed toxic-waste value of the synthetic test SRS
 
@@ -54,7 +56,19 @@ def parse():
     ap.add_argument("--inflight", type=int, default=2,
                     help="proofs in flight per GPU: independent provers (own stream + scratch, shared SRS), one host "
                          "thread each; a step is one batch of this many proofs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64), for comparing builds")
     return ap.parse_args()
+
+
+def dump_outputs(path, proofs):
+    """proofs: the 768-byte proof of every lane (Proof.to_bytes order: 24 big-endian 256-bit words).  Written as
+    proof.npy, shape (lanes, 24, 8): each word as eight 32-bit limbs, least significant first (exact in float64)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    words = np.frombuffer(b"".join(proofs), dtype=np.uint8).reshape(len(proofs), 24, 32)[:, :, ::-1]
+    limbs = np.ascontiguousarray(words).view("<u4")
+    np.save(os.path.join(path, "proof.npy"), limbs.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------------------------
@@ -369,15 +383,17 @@ def b200_arm(args):
         barrier()
     run_lanes(prove_device, args.warmup)
     barrier()
-    ref_proof = proof.raw
-    sampler.recording.set()  # sampling is already running during this last untimed step: nothing about it is new
-    run_lanes(prove_host, 1)  # to the driver when the timed region starts
-    assert all(lane["proof"].raw == ref_proof for lane in lanes), "lanes / host- and device-buffer paths disagree"
+    # sampling is already running during this last untimed step: nothing about it is new when the timed region starts
+    sampler.recording.set()
+    run_lanes(prove_host, 1)
+    ref_proof = proof.raw  # the device-buffer path is checked against it after its timed steps (last_proofs)
+    assert all(lane["proof"].raw == ref_proof for lane in lanes), "lanes disagree"
     torch.cuda.synchronize()
     sampler.samples.clear()
     launches0 = sum(lane["ctx"].launches for lane in lanes)
     ms_dev = timed(prove_device, args.steps)
     launches = sum(lane["ctx"].launches for lane in lanes) - launches0
+    last_proofs = [lane["proof"].raw for lane in lanes]  # the last timed step's results (--dump-outputs)
     ms_e2e = timed(prove_host, args.steps)
     # The device-resident path does strictly less than the host-buffer path.  A reading more than 25 % ABOVE it means the
     # first timed region was hit by a one-off stall (seen once on rank 0 of an 8-GPU run: 369 ms against 219 ms on the
@@ -388,10 +404,12 @@ def b200_arm(args):
         launches0 = sum(lane["ctx"].launches for lane in lanes)
         ms_dev = timed(prove_device, args.steps, name="prove_device (re-measured)")
         launches = sum(lane["ctx"].launches for lane in lanes) - launches0
+        last_proofs = [lane["proof"].raw for lane in lanes]
     sampler.recording.clear()
     sampler.stop_flag.set()
     sampler.join(timeout=2)
     assert all(lane["proof"].raw == ref_proof for lane in lanes)
+    assert all(p == ref_proof for p in last_proofs), "host- and device-buffer paths disagree"
     # per-kernel durations for the roofline: the same `steps` proofs on lane 0 alone with the library's event pairs
     # around every accumulation launch and NTT pass (alone, so that a duration is the kernel's own and not a share of
     # an SM array it divides with the other lane's kernels)
@@ -562,6 +580,8 @@ def b200_arm(args):
         verified = bool(vk.verify_proof(n, pf, pub_ints) and vk.verify_proof_unoptimized(n, pf, pub_ints)
                         and not vk.verify_proof(n, pb.Proof.from_bytes(bytes(bad)), pub_ints))
         assert verified, "the benchmarked proof does not verify"
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_proofs)
 
     if rank != 0:
         if world > 1:

@@ -43,6 +43,20 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_dump_outputs_holds_the_proof_words_exactly(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    import numpy as np
+    raw = bytes.fromhex(json.load(open(os.path.join(ROOT, "tests", "golden", "proof_2p20.json")))["proof_hex"])
+    other = bytes(reversed(raw))
+    bench.dump_outputs(str(tmp_path / "out"), [raw, other])
+    got = np.load(tmp_path / "out" / "proof.npy")
+    assert got.dtype == np.float64 and got.shape == (2, 24, 8)
+    for lane, proof in enumerate((raw, other)):
+        words = [sum(int(got[lane, k, i]) << (32 * i) for i in range(8)) for k in range(24)]
+        assert words == [int.from_bytes(proof[i:i + 32], "big") for i in range(0, 768, 32)]
+
+
 def test_cuda_arm_refuses_without_gpu():
     import torch
     if torch.cuda.is_available():

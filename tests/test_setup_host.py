@@ -1,18 +1,16 @@
 """CPU: host logic of plonkathon_b200/setup.py for the Lagrange-basis SRS (SURVEY 8(f) N4) -- the snarkjs section
-walker and the decoding of section 12 -- checked against the reference's ceremony file where it is mounted, and,
-everywhere, through properties of the committed fixture (tests/golden/ptau_lagrange_p0_p4.bin, the first 31 points
+walker and the decoding of section 12 -- checked against the section table of the reference's ceremony file, and
+through properties of the committed fixture (tests/golden/ptau_lagrange_p0_p4.bin, the first 31 points
 of that section): for every domain size the Lagrange points sum to the generator, and the size-8 block reproduces
 the reference's commitment KAT (test.py:23-28) with no inverse transform."""
+import hashlib
 import os
-
-import pytest
 
 from oracle import plonk_oracle as O
 from plonkathon_b200.setup import PTAU_SECTION_LAGRANGE_G1, decode_ptau_coordinates, ptau_sections
 from tests.golden_io import GOLDEN, PTAU_HEAD, load_json, pt
 
 FIXTURE = os.path.join(GOLDEN, "ptau_lagrange_p0_p4.bin")
-REAL = "/root/reference/test/powersOfTau28_hez_final_11.ptau"
 FACTOR = pow(2, 256, O.Q_MOD)
 
 
@@ -41,12 +39,22 @@ def test_section_walker_on_a_synthesised_file():
     assert ptau_sections(head) == {1: (24, 44), 2: (80, 262080)}
 
 
-@pytest.mark.skipif(not os.path.exists(REAL), reason="the reference tree is only mounted in the build container")
 def test_section_walker_on_the_reference_file():
-    contents = open(REAL, "rb").read()
-    secs = ptau_sections(contents)
+    """the reference's ceremony file rebuilt at full length from its recorded section table (reference_pins.json),
+    the committed head and the committed section-12 points; every other byte is zero"""
+    real = load_json("reference_pins.json")["ptau"]
+    contents = bytearray(real["length"])
+    head = open(PTAU_HEAD, "rb").read()
+    contents[:len(head)] = head
+    assert bytes(contents[:12]) == bytes.fromhex(real["head"])
+    for sid, pos, size in real["sections"]:
+        contents[pos:pos + 12] = sid.to_bytes(4, "little") + size.to_bytes(8, "little")
+    lag = open(FIXTURE, "rb").read()
+    contents[869812:869812 + len(lag)] = lag
+    secs = ptau_sections(bytes(contents))
+    assert secs == {sid: (pos + 12, size) for sid, pos, size in real["sections"]}
     assert secs[2] == (80, 262080) and secs[3][0] == 262172 and secs[12] == (869812, 64 * (2 ** 13 - 1))
-    assert contents[869812:869812 + 64 * 31] == open(FIXTURE, "rb").read()
+    assert hashlib.sha256(lag).hexdigest() == real["lagrange_p0_p4_sha256"]
 
 
 def test_lagrange_blocks_are_lagrange_bases():
