@@ -12,6 +12,9 @@
 // every 32x32->64 partial product lands on an aligned register pair; written as
 // mad.lo.cc / madc.hi.cc pairs, which ptxas fuses into one IMAD.WIDE.U32.X each
 // (136 IMAD-class instructions per product; checked with cuobjdump -sass).
+// Squarings and the two-product sums of the group law (A B + C D) instead build the 512-bit product(s)
+// with the same fused rows and reduce once (fp_sqr_wide / fp_mul_wide + fp_redc): 108 and 200
+// multiplier instructions against 136 and 272.
 //
 // Every PTX instruction is wrapped in a tiny function that has a host emulation with an explicit
 // carry flag, so the identical limb-level algorithm is unit-tested on the CPU
@@ -292,8 +295,230 @@ PB_HD Fp<P> fp_mul(const Fp<P>& a, const Fp<P>& b) {
 #endif
 }
 
+// ---- wide products and a separate Montgomery reduction ----------------------------------------------------------
+// A 512-bit product is accumulated in two arrays: E holds the partial products that start at an even limb position
+// (E[k] has weight 2^(32k)), O those that start at an odd one (O[k] has weight 2^(32(k+1))).  Every 64-bit partial
+// product lands on an aligned pair (2k, 2k+1) of one array, so each row is a mad.lo.cc / madc.hi.cc chain that
+// ptxas fuses into IMAD.WIDE.U32(.X), as in the CIOS product.  Unwritten limbs of E and O are zero.
+//
+// acc pairs (0,1) .. (2N-2,2N-1) += x[0] y, x[2] y, .., x[2N-2] y.
+//   TOP  : acc[2N-1] is still zero and the row cannot carry out of it (the caller's bound on the partial sum).
+//   else : the carry out of acc[2N-1] goes to acc[2N], which is still unwritten.
+template <int N, bool TOP>
+PB_HD void fp_wide_chain(uint32_t* acc, const uint32_t* x, uint32_t y) {
+  acc[0] = mad_lo_cc(x[0], y, acc[0]);
+#pragma unroll
+  for (int k = 0; k < N; k++) {
+    if (k > 0) acc[2 * k] = madc_lo_cc(x[2 * k], y, acc[2 * k]);
+    if (TOP && k == N - 1) acc[2 * k + 1] = madc_hi(x[2 * k], y, 0u);
+    else acc[2 * k + 1] = madc_hi_cc(x[2 * k], y, acc[2 * k + 1]);
+  }
+  if (!TOP) acc[2 * N] = addc(0u, 0u);
+}
+
+// E + 2^32 O = a * b (64 fused products).  Row i adds a * b_i at limb i; after row i the partial sum is below
+// 2^(256 + 32 (i + 1)), which is what makes the TOP rows safe: their top limb is limb 8 + i.
+PB_HD void fp_wide_rows(uint32_t* E, uint32_t* O, const uint32_t* a, const uint32_t* b) {
+#pragma unroll
+  for (int k = 0; k < 16; k++) { E[k] = 0; O[k] = 0; }
+#pragma unroll
+  for (int j = 0; j < 8; j += 2) {
+    E[j] = mul_lo(a[j], b[0]);
+    E[j + 1] = mul_hi(a[j], b[0]);
+    O[j] = mul_lo(a[j + 1], b[0]);
+    O[j + 1] = mul_hi(a[j + 1], b[0]);
+  }
+#pragma unroll
+  for (int i = 1; i < 8; i++) {
+    if (i & 1) {  // odd limbs of a land on even positions
+      fp_wide_chain<4, true>(E + i + 1, a + 1, b[i]);
+      fp_wide_chain<4, false>(O + i - 1, a, b[i]);
+    } else {
+      fp_wide_chain<4, false>(E + i, a, b[i]);
+      fp_wide_chain<4, true>(O + i, a + 1, b[i]);
+    }
+  }
+}
+
+// T (16 limbs) = a * b
 template <class P>
-PB_HD Fp<P> fp_sqr(const Fp<P>& a) { return fp_mul(a, a); }
+PB_HD void fp_mul_wide(uint32_t* T, const Fp<P>& a, const Fp<P>& b) {
+  uint32_t E[16], O[16];
+  fp_wide_rows(E, O, a.v, b.v);
+  T[0] = E[0];
+  T[1] = add_cc(E[1], O[0]);
+#pragma unroll
+  for (int k = 2; k < 15; k++) T[k] = addc_cc(E[k], O[k - 1]);
+  T[15] = addc(E[15], O[14]);  // a * b < 2^512: no carry out
+}
+
+// T (16 limbs) += a * b; returns the carry out of limb 15 (the 17th limb of the sum)
+template <class P>
+PB_HD uint32_t fp_mad_wide(uint32_t* T, const Fp<P>& a, const Fp<P>& b) {
+  uint32_t E[16], O[16];
+  fp_wide_rows(E, O, a.v, b.v);
+  T[0] = add_cc(T[0], E[0]);
+#pragma unroll
+  for (int k = 1; k < 15; k++) T[k] = addc_cc(T[k], E[k]);
+  T[15] = addc_cc(T[15], E[15]);
+  uint32_t c = addc(0u, 0u);
+  T[1] = add_cc(T[1], O[0]);
+#pragma unroll
+  for (int k = 2; k < 16; k++) T[k] = addc_cc(T[k], O[k - 1]);
+  return addc(c, 0u);
+}
+
+// T (16 limbs) = a^2: the 28 products a_i a_j (i < j) into E / O, doubled by a one-bit shift (their sum is below
+// a^2 / 2 < 2^511), then the 8 squares a_i^2 on the pairs (2i, 2i+1): 36 fused products instead of 64.
+template <class P>
+PB_HD void fp_sqr_wide(uint32_t* T, const Fp<P>& a) {
+  const uint32_t* x = a.v;
+  uint32_t E[16], O[16];
+#pragma unroll
+  for (int k = 0; k < 16; k++) { E[k] = 0; O[k] = 0; }
+  // row i: a_j a_i for j > i at position i + j; j - i odd -> O from index 2i, j - i even -> E from index 2i + 2
+#pragma unroll
+  for (int j = 1; j < 8; j += 2) {
+    O[j - 1] = mul_lo(x[j], x[0]);
+    O[j] = mul_hi(x[j], x[0]);
+  }
+#pragma unroll
+  for (int j = 2; j < 8; j += 2) {
+    E[j] = mul_lo(x[j], x[0]);
+    E[j + 1] = mul_hi(x[j], x[0]);
+  }
+  fp_wide_chain<3, false>(O + 2, x + 2, x[1]);
+  fp_wide_chain<3, true>(E + 4, x + 3, x[1]);
+  fp_wide_chain<3, true>(O + 4, x + 3, x[2]);
+  fp_wide_chain<2, false>(E + 6, x + 4, x[2]);
+  fp_wide_chain<2, false>(O + 6, x + 4, x[3]);
+  fp_wide_chain<2, true>(E + 8, x + 5, x[3]);
+  fp_wide_chain<2, true>(O + 8, x + 5, x[4]);
+  fp_wide_chain<1, false>(E + 10, x + 6, x[4]);
+  fp_wide_chain<1, false>(O + 10, x + 6, x[5]);
+  fp_wide_chain<1, true>(E + 12, x + 7, x[5]);
+  fp_wide_chain<1, true>(O + 12, x + 7, x[6]);
+  // D = E + 2^32 O (E[0] = E[1] = 0), then T = 2 D
+  uint32_t D[16];
+  D[0] = 0;
+  D[1] = O[0];
+  D[2] = add_cc(E[2], O[1]);
+#pragma unroll
+  for (int k = 3; k < 14; k++) D[k] = addc_cc(E[k], O[k - 1]);
+  D[14] = addc_cc(O[13], 0u);
+  D[15] = addc(0u, 0u);
+#pragma unroll
+  for (int k = 15; k > 0; k--) T[k] = (D[k] << 1) | (D[k - 1] >> 31);
+  T[0] = mad_lo_cc(x[0], x[0], 0u);
+  T[1] = madc_hi_cc(x[0], x[0], T[1]);
+#pragma unroll
+  for (int i = 1; i < 7; i++) {
+    T[2 * i] = madc_lo_cc(x[i], x[i], T[2 * i]);
+    T[2 * i + 1] = madc_hi_cc(x[i], x[i], T[2 * i + 1]);
+  }
+  T[14] = madc_lo_cc(x[7], x[7], T[14]);
+  T[15] = madc_hi(x[7], x[7], T[15]);  // a^2 < 2^512: no carry out
+}
+
+// One word of the reduction, with the CIOS step's state T = U + 2^32 * V + w.  On entry V is the accumulator the
+// previous step cleared (V[0] + w == 0 mod 2^32) and U the shifted one; dividing by 2^32 makes U aligned with
+// carry-in (w != 0), the pending word becomes V[1] and V >> 64 takes the shifted role.  Then m clears U's low word.
+//   FIRST: U = the low half of the input, V unused, w = 0.
+// The state stays below 2^256 + 2^32 p < 2^288, so nothing carries out of the shifted accumulator's top limb.
+template <class P, bool FIRST>
+PB_HD void fp_redc_step(uint32_t* U, uint32_t* V, uint32_t& w) {
+  uint32_t m;
+  if (FIRST) {
+    m = mul_lo(U[0], P::NP0);
+#pragma unroll
+    for (int j = 0; j < 8; j += 2) {
+      V[j] = mul_lo(P::p(j + 1), m);
+      V[j + 1] = mul_hi(P::p(j + 1), m);
+    }
+    fp_mad_row_mod<P, 0>(U, m);
+    w = 0;
+  } else {
+    const uint32_t wn = V[1];
+    (void)add_cc(w, 0xffffffffu);  // CF = (w != 0)
+    m = mul_lo(addc(U[0], wn), P::NP0);
+    V[0] = mad_lo_cc(P::p(1), m, V[2]);
+    V[1] = madc_hi_cc(P::p(1), m, V[3]);
+    V[2] = madc_lo_cc(P::p(3), m, V[4]);
+    V[3] = madc_hi_cc(P::p(3), m, V[5]);
+    V[4] = madc_lo_cc(P::p(5), m, V[6]);
+    V[5] = madc_hi_cc(P::p(5), m, V[7]);
+    V[6] = madc_lo_cc(P::p(7), m, 0u);
+    V[7] = madc_hi(P::p(7), m, 0u);
+    (void)add_cc(w, 0xffffffffu);
+    U[0] = madc_lo_cc(P::p(0), m, U[0]);
+    U[1] = madc_hi_cc(P::p(0), m, U[1]);
+#pragma unroll
+    for (int j = 2; j < 8; j += 2) {
+      U[j] = madc_lo_cc(P::p(j), m, U[j]);
+      U[j + 1] = madc_hi_cc(P::p(j), m, U[j + 1]);
+    }
+    w = wn;
+  }
+  V[7] = addc(V[7], 0u);  // carry out of U limb 7
+}
+
+// Montgomery reduction T R^-1 mod p of a 16-limb T < p 2^256, fully reduced.  The eight steps reduce the low half
+// to (T_lo + m p) / 2^256 <= p (m < 2^256); the high half T_hi < p is added after, and the sum is below 2p.
+// 72 multiplier instructions: 8 for the words m, 64 fused for m p.
+template <class P>
+PB_HD Fp<P> fp_redc(const uint32_t* T) {
+  uint32_t X[8], Y[8], w;
+#pragma unroll
+  for (int i = 0; i < 8; i++) X[i] = T[i];
+  fp_redc_step<P, true>(X, Y, w);
+  fp_redc_step<P, false>(Y, X, w);
+  fp_redc_step<P, false>(X, Y, w);
+  fp_redc_step<P, false>(Y, X, w);
+  fp_redc_step<P, false>(X, Y, w);
+  fp_redc_step<P, false>(Y, X, w);
+  fp_redc_step<P, false>(X, Y, w);
+  fp_redc_step<P, false>(Y, X, w);
+  // last step had U = Y, V = X:  (T_lo + m p) / 2^256 = X + (Y >> 32) + (w != 0)
+  Fp<P> r;
+  (void)add_cc(w, 0xffffffffu);
+  r.v[0] = addc_cc(X[0], Y[1]);
+#pragma unroll
+  for (int i = 1; i < 7; i++) r.v[i] = addc_cc(X[i], Y[i + 1]);
+  r.v[7] = addc(X[7], 0u);
+  r.v[0] = add_cc(r.v[0], T[8]);
+#pragma unroll
+  for (int i = 1; i < 7; i++) r.v[i] = addc_cc(r.v[i], T[8 + i]);
+  r.v[7] = addc(r.v[7], T[15]);
+  fp_reduce_once(r);
+  return r;
+}
+
+// a^2 R^-1 mod p: 108 multiplier instructions instead of the product's 136
+template <class P>
+PB_HD Fp<P> fp_sqr(const Fp<P>& a) {
+#if !defined(__CUDA_ARCH__) && defined(PB_HOST_FAST_MUL)
+  return fp_mul_host64(a, a);
+#else
+  uint32_t T[16];
+  fp_sqr_wide(T, a);
+  return fp_redc<P>(T);
+#endif
+}
+
+// (a b + c d) R^-1 mod p with one reduction, for the A B - C D shape of the group law (pass C and p - D).
+// a, b, c, d < p, so a b + c d < 2 p^2 < p 2^256 because 2p < 2^256: the reduction's input bound holds and the
+// 512-bit sum does not carry out.  200 multiplier instructions instead of two products' 272.
+template <class P>
+PB_HD Fp<P> fp_mul_sum2(const Fp<P>& a, const Fp<P>& b, const Fp<P>& c, const Fp<P>& d) {
+#if !defined(__CUDA_ARCH__) && defined(PB_HOST_FAST_MUL)
+  return fp_add(fp_mul_host64(a, b), fp_mul_host64(c, d));
+#else
+  uint32_t T[16];
+  fp_mul_wide(T, a, b);
+  (void)fp_mad_wide(T, c, d);
+  return fp_redc<P>(T);
+#endif
+}
 
 template <class P>
 PB_HD Fp<P> fp_to_mont(const Fp<P>& a) { return fp_mul(a, Fp<P>::r2()); }

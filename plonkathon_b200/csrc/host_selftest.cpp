@@ -1,6 +1,6 @@
 // Host build of the limb-level arithmetic in field.cuh / curve.cuh (same code path as the device,
 // PTX carry-chain primitives replaced by their emulation).  TEST INFRASTRUCTURE: loaded only by
-// tests/test_host_arith.py through ctypes; never linked into libplonk_b200.so.
+// tests/test_host_arith.py and tests/test_field_wide.py through ctypes; never linked into libplonk_b200.so.
 #include "field.cuh"
 #include "curve.cuh"
 #include "msm_digits.cuh"
@@ -38,6 +38,35 @@ int hs_field_op(int field, int op, const uint32_t* a, const uint32_t* b, uint32_
     st(out, r);                                                  \
   }
   if (field == 0) RUN(Fr) else RUN(Fq)
+  return 0;
+}
+
+// The wide-product building blocks of field.cuh.  a, b, c, d: 8 limbs each; t: 16 limbs; out: 16 limbs (ops 0, 1, 4)
+// or 8 (ops 2, 3).  op: 0 out = a b, 1 out = a^2, 2 out = redc(t), 3 out = (a b + c d) R^-1, 4 out = t + a b with the
+// carry limb as the return value ; field: 0 Fr, 1 Fq.  Returns -1 on a bad op.
+int hs_wide_op(int field, int op, const uint32_t* a, const uint32_t* b, const uint32_t* c, const uint32_t* d,
+               const uint32_t* t, uint32_t* out) {
+#define RUN_WIDE(F, P)                                                        \
+  {                                                                           \
+    F x = ld<F>(a), y = ld<F>(b), z = ld<F>(c), u = ld<F>(d);                 \
+    uint32_t T[16];                                                           \
+    memcpy(T, t, sizeof(T));                                                  \
+    switch (op) {                                                             \
+      case 0: fp_mul_wide(T, x, y); break;                                    \
+      case 1: fp_sqr_wide(T, x); break;                                       \
+      case 2: st(out, fp_redc<P>(T)); return 0;                               \
+      case 3: st(out, fp_mul_sum2(x, y, z, u)); return 0;                     \
+      case 4: {                                                               \
+        const uint32_t carry = fp_mad_wide(T, x, y);                          \
+        memcpy(out, T, sizeof(T));                                            \
+        return (int)carry;                                                    \
+      }                                                                       \
+      default: return -1;                                                     \
+    }                                                                         \
+    memcpy(out, T, sizeof(T));                                                \
+  }
+  if (field == 0) RUN_WIDE(Fr, FrParams) else RUN_WIDE(Fq, FqParams)
+#undef RUN_WIDE
   return 0;
 }
 

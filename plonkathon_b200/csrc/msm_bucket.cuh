@@ -288,7 +288,7 @@ PB_HD void g1_add_mixed_sel(G1XYZZ& acc, const G1Affine& p, bool take) {
   Fq PPP = fp_mul(Pd, PP);
   Fq Q = fp_mul(acc.X, PP);
   Fq X3 = fp_sub(fp_sub(fp_sqr(Rd), PPP), fp_dbl(Q));
-  Fq Y3 = fp_sub(fp_mul(Rd, fp_sub(Q, X3)), fp_mul(acc.Y, PPP));
+  Fq Y3 = fp_mul_sum2(Rd, fp_sub(Q, X3), acc.Y, fp_neg(PPP));
   Fq ZZ3 = fp_mul(acc.ZZ, PP);
   Fq ZZZ3 = fp_mul(acc.ZZZ, PPP);
   const Fq one = Fq::one();
